@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- placements/sec of the topology-aware GPU placement scorer.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], SURVEY.md 8(d) "C2"): 100,000 nodes x 10,000 pods, 8 GPUs per node,
@@ -29,6 +29,9 @@ Prints ONE JSON line on rank 0.  Beyond the base contract:
   multi_device_handle   (N > 1) rank 0 also scores C2 through ONE handle over all N devices
                         (kgpu_create(devs, N): in-library NCCL all-gather), keys compared.
   cpu_baseline    Oracle B (tuned C port, all host cores) on a bounded pod sample.
+`--dump-outputs DIR` (rank 0) writes the keys of the last timed step, unpacked as a caller does (scorer.unpack_key), to
+DIR/cost.npy, DIR/node_id.npy and DIR/gpu_mask.npy: float64[10000], exact (every field < 2**53); a pod without a fit
+(KGPU_NO_FIT) reads 0xFFFFFF / 0xFFFFFFFF / 0xFF.  The inputs are seeded, so two builds can be compared file for file.
 `--impl reference` times the CPU port of the path instead (the reference itself is Go with un-vendored
 dependencies and cannot be built here: DESIGN.md "Oracle").
 """
@@ -81,6 +84,14 @@ def kernel_source_sha() -> str:
         with open(os.path.join(ROOT, "kubegpu_b200", "csrc", f), "rb") as fh:
             h.update(fh.read())
     return h.hexdigest()[:12]
+
+
+def dump_keys(out_dir: str, keys: np.ndarray) -> None:
+    """--dump-outputs: the per-pod keys as the three fields a caller unpacks, float64 (lossless)."""
+    os.makedirs(out_dir, exist_ok=True)
+    fields = {"cost": keys >> np.uint64(40), "node_id": (keys >> np.uint64(8)) & np.uint64(0xFFFFFFFF), "gpu_mask": keys & np.uint64(0xFF)}
+    for name, a in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def committed_counts():
@@ -276,7 +287,12 @@ def main():
                     help="multi-GPU key exchange: peer-memory push kernel (auto when it connects), NCCL all-gather + K2, "
                          "or one NCCL all-reduce(min)")
     ap.add_argument("--graph", action="store_true", help="replay the NCCL-path step as one CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the keys of the last timed step to DIR/*.npy (kgpu arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the kgpu arm")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -303,7 +319,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
         host_group = dist.new_group(backend="gloo")            # host-side barriers: waiting ranks must not spin on their GPU
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
     peak, peak_src = measured_peak_gbs()
     props = torch.cuda.get_device_properties(local_rank)
     stream = torch.cuda.Stream(device=dev)          # everything (K1, exchange, copies) is enqueued here
@@ -385,8 +401,11 @@ def main():
             return final
         return local
 
+    last_keys = [None]                              # the tensor the last (or the graph-captured) step left its keys in
+
     def step_device():
-        return step_on(scorer, d_pods, N_PODS, d_local, d_gather, d_final)
+        last_keys[0] = step_on(scorer, d_pods, N_PODS, d_local, d_gather, d_final)
+        return last_keys[0]
 
     def step_e2e():
         """host pods -> host keys through the public call."""
@@ -432,8 +451,9 @@ def main():
     sampler.start()
     total_ms = timed(graph.replay if graph is not None else step_device, K)
     gpu_launches = scorer.kernel_launches - launches0 if graph is None else K * (scorer.kernel_launches - launches_before_capture)
-    final_dev = step_device() if graph is None else d_final    # the keys of the timed computation, kept for the parity gate
-    timed_keys = final_dev.cpu().numpy().view(np.uint64).copy()
+    timed_keys = last_keys[0].cpu().numpy().view(np.uint64).copy()   # the last timed step's keys, kept for the parity gate
+    if rank == 0 and args.dump_outputs:
+        dump_keys(args.dump_outputs, timed_keys)
     # kernel only (no exchange): K1s launch(es) on this rank's shard
     k1_total_ms = timed(lambda: scorer.score_batch_device(d_pods.data_ptr(), N_PODS, d_local.data_ptr(), stream.cuda_stream,
                                                           _lib.BATCH_NO_MIN_MEM), K)

@@ -4,6 +4,7 @@ import ctypes
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -46,15 +47,15 @@ def test_version_and_error_path_without_device(built_lib):
     assert L.kgpu_num_nodes(None) == 0 and L.kgpu_destroy(None) == _lib.OK
 
 
-def test_no_cpu_fallback_without_cuda():
-    """Product rule: without a CUDA device creating a scorer fails loudly."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
-    from kubegpu_b200.scorer import KgpuError, Scorer
-    with pytest.raises(KgpuError) as e:
-        Scorer()
-    assert e.value.code == _lib.ERR_CUDA and "no CPU path" in str(e.value)
+def test_no_cpu_fallback_without_cuda(built_lib):
+    """Product rule: without a CUDA device creating a scorer fails loudly.  A fresh process with every device
+    hidden, so the rule is checked on a machine with a GPU too."""
+    code = ("from kubegpu_b200.scorer import KgpuError, Scorer\n"
+            "try:\n    Scorer()\nexcept KgpuError as e:\n    print(e.code, e)\n")
+    out = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=120,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert out.stdout.startswith("%d " % _lib.ERR_CUDA) and "no CPU path" in out.stdout, out.stdout
 
 
 def test_product_does_not_touch_oracle():

@@ -32,23 +32,14 @@ def _inputs(tmp_path, N=1500, P=96):
     return topo, free, pods
 
 
-def _has_gpu():
-    try:
-        import torch
-        return torch.cuda.is_available()
-    except Exception:
-        return False
-
-
 def test_c99_program_builds_and_fails_loudly_without_gpu(tmp_path):
     if not os.path.exists(os.path.join(LIBDIR, "libkgpu.so")):
         pytest.skip("libkgpu.so not built")
     exe = _build(tmp_path)
-    if _has_gpu():
-        pytest.skip("a GPU is present: covered by the gpu test")
     topo, free, pods = _inputs(tmp_path, N=64, P=8)
     r = subprocess.run([exe, str(tmp_path / "topo.bin"), str(tmp_path / "free.bin"), str(tmp_path / "pods.bin"), "64", "8",
-                        str(tmp_path / "out.bin")], capture_output=True, text=True, timeout=120)
+                        str(tmp_path / "out.bin")], capture_output=True, text=True, timeout=120,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))      # no device, also on a machine that has one
     assert r.returncode == 3, (r.returncode, r.stderr)
     assert "no usable CUDA device" in r.stderr and not os.path.exists(tmp_path / "out.bin")
 
